@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mpts/s of one full MapEval metric pass (AC + CD + full CD + MME + voxel Gaussians + AWD + SCS).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C3] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic cloud pair (SURVEY.md §8d): both lattices are laid out from
 the fp64 clouds, NN est->gt and gt->est with the five-threshold accumulators and the full-Chamfer sums, MME of the
@@ -197,6 +197,28 @@ def _alloc_pinned(t):
     return t.pin_memory()
 
 
+def _dump_outputs(out_dir, res):
+    """Writes the result structs of one pass as DIR/<struct>.<field>.npy, one float64 array per field (the integer
+    counts are exact in float64).  The clouds are generated from fixed seeds, so two builds run with the same arguments
+    can be compared file by file."""
+    outs = {"nn": A.struct_to_dict(res["nn"]), "n_far": list(res["n_far"])}
+    for m, side in zip(res["mme"], ("est", "gt")):
+        outs[f"mme_{side}"] = A.struct_to_dict(m)
+    if res["awd"] is not None:
+        outs["awd"] = A.struct_to_dict(res["awd"])
+    os.makedirs(out_dir, exist_ok=True)
+
+    def write(name, v):
+        if isinstance(v, dict):
+            for k, x in v.items():
+                write(f"{name}.{k}", x)
+        else:
+            np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+    for name, v in outs.items():
+        write(name, v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -211,7 +233,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer arms (large configs on small hosts)")
     ap.add_argument("--gen", default="auto", choices=["auto", "numpy", "device"],
                     help="where the synthetic clouds are generated (auto: on the device above 20 M points)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the device-resident arm returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm only")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
@@ -366,6 +394,7 @@ def main():
         one_pass("device")
     stage_ms = {}
     ms_dev, launches, t0, t1 = timed("device", args.steps, stage_ms)
+    device_results = dict(results)      # the e2e arms below overwrite `results`
     t_last = t1
     ms_e2e = ms_page = None
     if do_e2e:
@@ -471,6 +500,8 @@ def main():
                                     "host_memory": "pageable (plain numpy arrays handed to me_set_cloud, the way a "
                                                    "std::vector<Eigen::Vector3d> caller does)"}
         os.write(real_stdout, (json.dumps(line) + "\n").encode())
+        if args.dump_outputs:
+            _dump_outputs(args.dump_outputs, device_results)
     ctx.close()
     if world > 1:
         dist.destroy_process_group()

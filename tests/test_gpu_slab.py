@@ -249,15 +249,15 @@ def test_sparse_cell_table_stays_replicated(api):
     """A scene that gets the sparse cell table (laid out whole) ignores the slab request: same results, replicated layout."""
     est, gt, cfg = synth.make_pair("C4", scale=0.004)
     p = A.make_nn_params(cfg["tau"], 1.0)
-    ref = _reference(api, est, gt, p, cfg["nn_radius"], cfg["vmd_voxel_size"], 20)
+    sparse = dict(max_grid_cells=1)         # a budget of one cell: this small scene would otherwise get a dense table
+    ref = _reference(api, est, gt, p, cfg["nn_radius"], cfg["vmd_voxel_size"], 20, **sparse)
     tot = 0
     for r in range(2):
-        with api.MapEvalB200(rank=r, world=2, vmd_voxel_size=cfg["vmd_voxel_size"]) as ctx:
+        with api.MapEvalB200(rank=r, world=2, vmd_voxel_size=cfg["vmd_voxel_size"], **sparse) as ctx:
             ctx.set_layout(A.ME_LAYOUT_SLAB)
             ctx.set_cloud(EST, est)
             ctx.set_cloud(GT, gt)
             e, g = ctx.eval_nn_accum(p)
-            if ctx.layout_active()["layout"] != A.ME_LAYOUT_REPLICATED:
-                pytest.skip("this scene got a dense table")
+            assert ctx.layout_active()["layout"] == A.ME_LAYOUT_REPLICATED
             tot += e.n_inlier[0]
     assert tot == ref["e"].n_inlier[0]

@@ -353,14 +353,11 @@ def test_map_eval_two_gpus_matches_one(exe, tmp_path):
         assert len(a) > 200 and a == b, name
 
 
-REF_CONFIG_DIR = "/root/reference/map_eval/config"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_CONFIG_DIR), reason="the reference checkout is only present in the authoring container")
 @pytest.mark.parametrize("name", ["config.yaml", "config_building_day.yaml", "config_corridor.yaml", "config_geode.yaml"])
-def test_loader_reads_the_references_shipped_configs(exe, name):
-    """The YAML-subset loader on the configuration files the reference ships (map_eval/config/*.yaml), unmodified."""
-    out, kv = _dump(exe, os.path.join(REF_CONFIG_DIR, name))
+def test_loader_reads_the_references_shipped_configs(exe, golden_dir, name):
+    """The YAML-subset loader on the configuration files the reference ships (map_eval/config/*.yaml), unmodified
+    (copies under tests/golden/reference_config/)."""
+    out, kv = _dump(exe, os.path.join(golden_dir, "reference_config", name))
     assert out.returncode == 0, out.stderr
     assert kv["registration_methods"] == "2" and float(kv["icp_max_distance"]) == 1.0
     assert [float(x) for x in kv["accuracy_level"].split(",")] == [0.2, 0.1, 0.08, 0.05, 0.01]

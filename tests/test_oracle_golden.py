@@ -1,6 +1,7 @@
 """Pins the oracle against the only known-answer artefacts the reference ships (SURVEY.md §4):
 the sample voxel_errors.txt / voxel_wasserstein_cdf.txt and the README run log of the same run."""
 import json
+import lzma
 import os
 
 import numpy as np
@@ -9,10 +10,11 @@ from oracle import oracle as O
 
 
 def _load(golden_dir):
-    z = np.load(os.path.join(golden_dir, "voxel_fixture.npz"))
+    rows = np.loadtxt(lzma.open(os.path.join(golden_dir, "voxel_errors.txt.xz"), "rt"))
+    cdf = np.loadtxt(lzma.open(os.path.join(golden_dir, "voxel_wasserstein_cdf.txt.xz"), "rt"))
     with open(os.path.join(golden_dir, "readme_run_log.json")) as f:
         log = json.load(f)
-    return z["rows"], z["cdf"], log
+    return rows, cdf, log
 
 
 def _sym(tri):
